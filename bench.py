@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # B200 engine (this repo)
     python bench.py --impl reference --gpus N ...            # CPU reference arm (oracle port, rank 0)
     python bench.py --workload {db5-shaped,db5-testset,large,train} ...
+    python bench.py ... --dump-outputs DIR                  # also write the last timed step's outputs as DIR/<name>.npy
 
 Workloads (BASELINE.json configs):
   db5-shaped   (headline, north_star / configs[1] shape) synthetic DB5.5-shaped residue graphs, 200+200 residues, k=10,
@@ -431,6 +432,37 @@ def timed_reps(torch, D: Dist, reps: int, body):
     return rep_ms, med, per_rank[med]
 
 
+OUTPUT_NAMES = ('ligand_coors', 'keypts_ligand', 'keypts_receptor', 'rotation', 'translation')
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, result, limit: int = DUMP_LIMIT_BYTES):
+    """Writes one step's result -- the model's 5-tuple of per-pair lists -- as out_dir/<name>.npy: the ligand coordinates
+    of all pairs concatenated in pair order, the other outputs stacked.  float64 outputs stay float64, the others are
+    written as float32.  Where the whole result exceeds `limit` bytes, a fixed random subset of the pairs (seed 0, kept
+    in pair order) that fits is written instead, so that two runs with the same arguments write the same pairs."""
+    import torch
+    n_lig = np.array([c.shape[0] for c in result[0]])
+    host = {'ligand_coors': torch.cat(result[0]).cpu().numpy()}
+    host.update({k: torch.stack(v).cpu().numpy() for k, v in zip(OUTPUT_NAMES[1:], result[1:])})
+    host = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32, copy=False) for k, v in host.items()}
+    lig = host['ligand_coors']
+    pair_bytes = n_lig * lig.itemsize * lig.shape[1] + sum(host[k][0].nbytes for k in OUTPUT_NAMES[1:])
+    keep = np.arange(len(n_lig))
+    if pair_bytes.sum() > limit:
+        order = np.random.default_rng(0).permutation(len(n_lig))
+        keep = np.sort(order[np.cumsum(pair_bytes[order]) <= limit])
+        start = np.concatenate([[0], np.cumsum(n_lig)[:-1]])
+        rows = np.concatenate([np.arange(start[i], start[i] + n_lig[i]) for i in keep]) if len(keep) else []
+        host = {k: (v[rows] if k == 'ligand_coors' else v[keep]) for k, v in host.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, f'{k}.npy'), v)
+    print(f'bench: wrote the last timed step\'s outputs of {len(keep)} of {len(n_lig)} pairs to {out_dir}',
+          file=sys.stderr, flush=True)
+    return keep
+
+
 def run_engine(args, rank, local_rank, world):
     numa = bind_to_gpu_numa(local_rank) if not args.no_numa_bind else None
     import torch
@@ -467,7 +499,10 @@ def run_engine(args, rank, local_rank, world):
     else:
         launch = lambda i: model.forward_async(dev_batches[i & 1], 0)
 
+    last = None
+
     def value_body():
+        nonlocal last
         pending = None
         for i in range(K):          # step i is launched before step i-1's status words are read
             nxt = launch(i)
@@ -475,6 +510,7 @@ def run_engine(args, rank, local_rank, world):
                 pending.result()
             pending = nxt
         pending.result()
+        last = pending
 
     for _ in range(W):
         launch(0).result()
@@ -488,6 +524,11 @@ def run_engine(args, rank, local_rank, world):
     rep_ms, med, per_rank_ms = timed_reps(torch, D, R, value_body)
     ms_total = rep_ms[med]
     value = total_pairs * K / (ms_total * 1e-3)
+    # The loop keeps only the last step's handle: holding its result (~2000 tensor views) across repetitions moved one
+    # of the interpreter's full garbage collections (~33 ms) into the timed window of the default run.  result()
+    # re-reads that step's output buffers, so it must run before anything is launched again.
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f'rank{rank}'), last.result())
 
     # ---- instrumented pass: the same K steps on the eager path with CUDA events around every edge / node stage ------
     timer = engine_mod.NativeStageTimer()
@@ -680,7 +721,15 @@ def main():
     ap.add_argument('--no-residue-e2e', action='store_true')
     ap.add_argument('--watchdog-seconds', type=int, default=1500,
                     help='abort (with a stack dump) instead of stalling forever if the run has not finished by then')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32 / float64, '
+                         'at most 64 MB: a fixed sample of the pairs beyond that); with several ranks, DIR/rank<r>/')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl == 'reference' or args.workload == 'train'):
+        ap.error('--dump-outputs needs an inference workload of the engine arm: the train workload updates the weights '
+                 'during a clock-timed lead-in, so its last step is not reproducible, and the reference arm keeps no outputs')
     if args.pairs_per_gpu <= 0:
         args.pairs_per_gpu = WORKLOADS[args.workload]['pairs_per_gpu']
     if args.watchdog_seconds > 0:
