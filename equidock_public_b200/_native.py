@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # EQD_LIB_PATH: load another build of the same ABI instead (A/B runs of kernel variants, scripts/forward_ab.py)
 LIB_PATH = os.environ.get('EQD_LIB_PATH') or os.path.join(_HERE, 'libeqd_iegmn.so')
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 EDGE_FEATS, N_RBF, HID, H0, H0_PAD, N_RES_TYPES, HEADS, TILE_ROWS = 27, 15, 64, 69, 72, 21, 50, 128
 STATUS_SVD_DEGENERATE, STATUS_NAN, STATUS_DEGREE_OVERFLOW, STATUS_BAD_RESIDUE = 1, 2, 4, 8
 
@@ -57,8 +57,13 @@ class EqdHeadParams(C.Structure):
     _fields_ = [('w_mean', _vp), ('b_mean', _vp), ('w_key', _vp), ('w_query', _vp), ('m_qk', _vp), ('leaky_slope', _f32)]
 
 
+class EqdDropout(C.Structure):
+    """eqd_dropout: counter-based dropout masks of a training forward / backward (key in DEVICE memory)."""
+    _fields_ = [('key', _vp), ('threshold', C.c_uint32), ('scale', _f32), ('rank', C.c_uint32)]
+
+
 # symbol -> (restype, argtypes); every symbol include/eqd_iegmn.h declares must be listed here
-_G, _L, _H = C.POINTER(EqdGraph), C.POINTER(EqdLayer), C.POINTER(EqdHeadParams)
+_G, _L, _H, _D = C.POINTER(EqdGraph), C.POINTER(EqdLayer), C.POINTER(EqdHeadParams), C.POINTER(EqdDropout)
 PROTOTYPES = {
     'eqd_abi_version': (C.c_int, []),
     'eqd_workspace_bytes': (C.c_size_t, [_i32, _i32, _i32]),
@@ -82,19 +87,25 @@ PROTOTYPES = {
     'eqd_head_fold': (C.c_int, [_H, _vp, _vp]),
     'eqd_forward_workspace_bytes': (C.c_size_t, [_G]),
     'eqd_iegmn_forward': (C.c_int, [_G, C.POINTER(_L), _i32, _H, C.POINTER(EqdForwardIO), _vp, C.c_size_t, _vp]),
+    'eqd_iegmn_forward_dropout': (C.c_int, [_G, C.POINTER(_L), _i32, _H, C.POINTER(EqdForwardIO), _D, _vp, C.c_size_t, _vp]),
+    'eqd_dropout_mask': (C.c_int, [_D, _i32, _i32, _i32, _i32, _vp, _vp]),
     'eqd_forward_stash_bytes': (C.c_size_t, [_G, _i32]),
     'eqd_forward_stash_offsets': (C.c_int, [_G, _i32, C.POINTER(C.c_size_t)]),
     'eqd_tn_partial_floats': (C.c_size_t, [C.c_int64, _i32, _i32, C.POINTER(_i32), C.POINTER(_i32)]),
     'eqd_tn_gemm': (C.c_int, [_vp, _i32, _i32, _vp, _i32, _i32, C.c_int64, _f32, _vp, _vp, C.POINTER(_i32), _vp]),
     'eqd_grad_reduce': (C.c_int, [_vp, _i32, C.c_int64, _vp, _vp, _i32, _vp, _vp]),
     'eqd_bwd_node_mlp': (C.c_int, [_G, _L] + [_vp] * 3 + [_i32, _vp, _vp, _i32] + [_vp] * 9 + [C.POINTER(_i32), _vp]),
+    'eqd_bwd_node_mlp_dropout': (C.c_int, [_G, _L] + [_vp] * 3 + [_i32, _vp, _vp, _i32] + [_vp] * 9 +
+                                 [C.POINTER(_i32), _D, _i32, _vp]),
     'eqd_bwd_attention': (C.c_int, [_G, _L, _vp, _vp, _i32, _vp, _vp, _vp, _vp]),
     'eqd_bwd_edge': (C.c_int, [_G, _L] + [_vp] * 14 + [C.POINTER(_i32), _vp]),
+    'eqd_bwd_edge_dropout': (C.c_int, [_G, _L] + [_vp] * 14 + [C.POINTER(_i32), _D, _i32, _vp]),
     'eqd_bwd_edge_gather': (C.c_int, [_G, _vp, _vp, _vp, _vp, _vp, _f32, _vp, _i32, _vp, _vp]),
     'eqd_bwd_project': (C.c_int, [_G, _L, _vp, _vp, _vp, _vp]),
     'eqd_bwd_embed': (C.c_int, [_G, _vp, _vp, _vp, _vp, _vp, _vp]),
     'eqd_bwd_head_workspace_bytes': (C.c_size_t, [_i32, _i32, _i32]),
     'eqd_bwd_head': (C.c_int, [_G, _H] + [_vp] * 9 + [C.c_size_t] + [_vp] * 6),
+    'eqd_bwd_head_dropout': (C.c_int, [_G, _H] + [_vp] * 9 + [C.c_size_t] + [_vp] * 5 + [_D, _i32, _vp]),
     'eqd_losses_workspace_bytes': (C.c_size_t, [_i32, _i32]),
     'eqd_losses': (C.c_int, [_G] + [_vp] * 7 + [_i32, _i32, _f32, _f32, _f32, _f32, _vp, C.c_size_t] + [_vp] * 6),
     'eqd_graph_build_workspace_bytes': (C.c_size_t, [_i32]),
@@ -150,3 +161,30 @@ def ptr(t):
     if t is None:
         return None
     return C.c_void_p(t.data_ptr())
+
+
+def dropout_threshold(p: float) -> int:
+    """Keep iff the Philox word >= this: min(round(p 2^32), 2^32 - 1) (include/eqd_iegmn.h, eqd_dropout)."""
+    return min(int(round(float(p) * 2.0 ** 32)), 2 ** 32 - 1)
+
+
+def dropout_scale(p: float) -> float:
+    """fp32(1 / (1 - p)), the factor of a kept element (torch.nn.Dropout's)."""
+    return float(C.c_float(1.0 / (1.0 - float(p))).value)
+
+
+class Dropout:
+    """The dropout state of ONE forward: probability, the 64-bit key (a one-element int64 DEVICE tensor drawn from torch's CUDA
+    generator on the device: no host sync, reproducible under ``torch.manual_seed``, the CPU generator untouched) and the
+    data-parallel rank.  ``struct`` is the eqd_dropout descriptor the entry points take; the backward passes the same one."""
+
+    def __init__(self, p: float, device, rank: int = 0, key=None):
+        p = float(p)
+        if not 0.0 < p < 1.0:
+            raise ValueError(f'dropout probability {p} outside (0, 1)')
+        self.p, self.rank = p, int(rank)
+        if key is None:
+            import torch
+            key = torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=device)
+        self.key = key
+        self.struct = EqdDropout(key.data_ptr(), dropout_threshold(p), dropout_scale(p), self.rank)

@@ -13,6 +13,7 @@
 // over IN-edges, dx = (1 - eta) dx' + sum_out dx_rel - sum_in dx_rel: fixed summation order, no atomics.
 // Restated in oracle/backward_manual.py::edge_bwd / edge_gather.
 #include "bwd_common.cuh"
+#include "dropout.cuh"
 
 namespace eqd {
 
@@ -37,12 +38,16 @@ struct EdgeBwdSmem {
   int src[EQD_TM], dst[EQD_TM];
 };
 
+// DROPOUT: the forward's site-0 / site-1 masks (c2 = drop.c2, drop.c2 + 1) are regenerated per (row, column group):
+// a1 = m s lrelu(z1), dz1 = m s lrelu'(z1) da;  c3 = m s lrelu(z3) (phi, dw4), dz3 = m s lrelu'(z3) dphi w4.
+template <bool DROPOUT>
 __global__ void __launch_bounds__(EQD_THREADS)
 bwd_edge_kernel(eqd_graph g, eqd_layer_params p, const float* __restrict__ w2lin, const float* __restrict__ w3lin,
                 const float* __restrict__ proj, const double* __restrict__ x_in, const float* __restrict__ daggr,
                 const double* __restrict__ dx_out, float* __restrict__ ein_out, float* __restrict__ n1_out,
                 float* __restrict__ msg_out, float* __restrict__ dz3_out, float* __restrict__ dmsg_out,
-                float* __restrict__ dz1_out, double* __restrict__ dxrel_out, float* __restrict__ vec_partial) {
+                float* __restrict__ dz1_out, double* __restrict__ dxrel_out, float* __restrict__ vec_partial,
+                DropoutArgs drop) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   EdgeBwdSmem& s = *reinterpret_cast<EdgeBwdSmem*>(smem_raw);
   const int tid = threadIdx.x, ty = tid >> 3, tx = tid & 7;
@@ -147,15 +152,22 @@ bwd_edge_kernel(eqd_graph g, eqd_layer_params p, const float* __restrict__ w2lin
       }
     }
     gemm_nn<false>(acc, accx, s.bufE + ty * 8 * BE_LD1, BE_LD1, s.w1, 64, BE_K1, tx);
-    unsigned pos_lo = 0, pos_hi = 0;
+    unsigned pos_lo = 0, pos_hi = 0, keep_lo = 0, keep_hi = 0;   // keep: site-0 mask bits, same layout as pos
     float nrm[8][8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
       float sum = 0.f;
+      if (DROPOUT) {   // columns col_nn(tx, 0..7) = 4 tx + 0..3, 32 + 4 tx + 0..3
+        const unsigned long long key = dropout_key(drop);
+        const unsigned row = (unsigned)(e0 + ty * 8 + i);
+        const unsigned k = dropout_keep4(drop, key, tx, row, drop.c2) | (dropout_keep4(drop, key, 8 + tx, row, drop.c2) << 4);
+        if (i < 4) keep_lo |= k << (i * 8); else keep_hi |= k << ((i - 4) * 8);
+      }
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         float a = lrelu(acc[i][j], slope);
         if (a > 0.f) { if (i < 4) pos_lo |= 1u << (i * 8 + j); else pos_hi |= 1u << ((i - 4) * 8 + j); }
+        if (DROPOUT) a *= dropout_mul(i < 4 ? keep_lo : keep_hi, (i & 3) * 8 + j, drop.scale);
         acc[i][j] = a;
         sum += a;
       }
@@ -198,12 +210,26 @@ bwd_edge_kernel(eqd_graph g, eqd_layer_params p, const float* __restrict__ w2lin
         const int r = ty * 8 + i;
         const float dph = s.dphi[r];
         float v = 0.f;
+        unsigned keep = 0;
+        if (DROPOUT) {
+          const unsigned long long key = dropout_key(drop);
+          const unsigned row = (unsigned)(e0 + r);
+          keep = dropout_keep4(drop, key, tx, row, drop.c2 + 1) | (dropout_keep4(drop, key, 8 + tx, row, drop.c2 + 1) << 4);
+        }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const float c3 = lrelu(acc[i][j], slope);
-          v = fmaf(c3, w4r[j], v);
-          w4sum[j] = fmaf(c3, dph, w4sum[j]);
-          acc[i][j] = dph * w4r[j] * lrelu_grad_from_post(c3, slope);     // dz3
+          if (DROPOUT) {
+            const float m = dropout_mul(keep, j, drop.scale);
+            const float c3m = c3 * m;
+            v = fmaf(c3m, w4r[j], v);
+            w4sum[j] = fmaf(c3m, dph, w4sum[j]);
+            acc[i][j] = dph * w4r[j] * lrelu_grad_from_post(c3, slope) * m;   // dz3
+          } else {
+            v = fmaf(c3, w4r[j], v);
+            w4sum[j] = fmaf(c3, dph, w4sum[j]);
+            acc[i][j] = dph * w4r[j] * lrelu_grad_from_post(c3, slope);     // dz3
+          }
         }
         v = row_sum8(v);
         if (tx == 0) s.phi[r] = v + p.b_coor2;
@@ -262,6 +288,7 @@ bwd_edge_kernel(eqd_graph g, eqd_layer_params p, const float* __restrict__ w2lin
       for (int j = 0; j < 8; ++j) {
         const bool pos = i < 4 ? (pos_lo >> (i * 8 + j)) & 1u : (pos_hi >> ((i - 4) * 8 + j)) & 1u;
         acc[i][j] = rstd * (acc[i][j] - m1 - nhat[j] * m2) * (pos ? 1.f : slope);
+        if (DROPOUT) acc[i][j] *= dropout_mul(i < 4 ? keep_lo : keep_hi, (i & 3) * 8 + j, drop.scale);
       }
     }
     __syncthreads();   // bufA (dmsg) no longer read
@@ -344,6 +371,17 @@ extern "C" int eqd_bwd_edge(const eqd_graph* g, const eqd_layer* p_l, const floa
                             const float* proj, const double* x_in, const float* daggr, const double* dx_out,
                             float* ein_out, float* n1_out, float* msg_out, float* dz3_out, float* dmsg_out, float* dz1_out,
                             double* dxrel_out, float* vec_partial, int32_t* n_partials_out, void* stream) {
+  return eqd_bwd_edge_dropout(g, p_l, w2lin, w3lin, proj, x_in, daggr, dx_out, ein_out, n1_out, msg_out, dz3_out, dmsg_out,
+                              dz1_out, dxrel_out, vec_partial, n_partials_out, nullptr, 0, stream);
+}
+
+extern "C" int eqd_bwd_edge_dropout(const eqd_graph* g, const eqd_layer* p_l, const float* w2lin, const float* w3lin,
+                                    const float* proj, const double* x_in, const float* daggr, const double* dx_out,
+                                    float* ein_out, float* n1_out, float* msg_out, float* dz3_out, float* dmsg_out,
+                                    float* dz1_out, double* dxrel_out, float* vec_partial, int32_t* n_partials_out,
+                                    const eqd_dropout* dropout, int32_t layer, void* stream) {
+  eqd::DropoutArgs d{};
+  if (const int rc = eqd::dropout_args(dropout, layer, 0, &d)) return rc;
   const eqd_layer_params* p = p_l ? &p_l->dev : nullptr;
   if (!g || !p || !w2lin || !w3lin || !proj || !x_in || !daggr || !dx_out || !ein_out || !n1_out || !msg_out || !dz3_out ||
       !dmsg_out || !dz1_out || !dxrel_out || !vec_partial)
@@ -354,10 +392,17 @@ extern "C" int eqd_bwd_edge(const eqd_graph* g, const eqd_layer* p_l, const floa
   if (n_partials_out) *n_partials_out = grid > 0 ? grid : 0;
   if (g->n_edges <= 0) return EQD_OK;
   size_t smem = sizeof(eqd::EdgeBwdSmem);
-  EQD_SET_SMEM((eqd::bwd_edge_kernel), smem);
-  eqd::bwd_edge_kernel<<<grid, EQD_THREADS, smem, (cudaStream_t)stream>>>(*g, *p, w2lin, w3lin, proj, x_in, daggr, dx_out,
-                                                                         ein_out, n1_out, msg_out, dz3_out, dmsg_out,
-                                                                         dz1_out, dxrel_out, vec_partial);
+  if (dropout) {
+    EQD_SET_SMEM((eqd::bwd_edge_kernel<true>), smem);
+    eqd::bwd_edge_kernel<true><<<grid, EQD_THREADS, smem, (cudaStream_t)stream>>>(
+        *g, *p, w2lin, w3lin, proj, x_in, daggr, dx_out, ein_out, n1_out, msg_out, dz3_out, dmsg_out, dz1_out, dxrel_out,
+        vec_partial, d);
+  } else {
+    EQD_SET_SMEM((eqd::bwd_edge_kernel<false>), smem);
+    eqd::bwd_edge_kernel<false><<<grid, EQD_THREADS, smem, (cudaStream_t)stream>>>(
+        *g, *p, w2lin, w3lin, proj, x_in, daggr, dx_out, ein_out, n1_out, msg_out, dz3_out, dmsg_out, dz1_out, dxrel_out,
+        vec_partial, d);
+  }
   EQD_CUDA_LAUNCH_CHECK();
   return EQD_OK;
 }

@@ -8,6 +8,7 @@
 // operands of the weight-gradient reductions (n5 = LN output, du) plus per-CTA partials of dgamma / dbeta.
 // Restated in oracle/backward_manual.py::node_mlp_bwd.
 #include "bwd_common.cuh"
+#include "dropout.cuh"
 
 namespace eqd {
 
@@ -20,14 +21,17 @@ struct NodeBwdCfg {
   static constexpr size_t SMEM = (size_t)(3 * BUF + WB + 16 * 64 + EQD_TM) * sizeof(float);
 };
 
-template <bool EXTRA>
+// DROPOUT: the forward's site-2 mask (c2 = drop.c2) regenerated per (node, column group): a5 = m s lrelu(u5),
+// du = m s lrelu'(u5) da.
+template <bool EXTRA, bool DROPOUT>
 __global__ void __launch_bounds__(EQD_THREADS)
 bwd_node_mlp_kernel(int n_nodes, eqd_layer_params p, const float* __restrict__ w_node1_lin /*[dhp][2dhp+136]*/,
                     const float* __restrict__ w_node2_lin /*[64][dhp]*/, const float* __restrict__ h_in, int ldh,
                     const float* __restrict__ aggr, const float* __restrict__ mu, int ldmu,
                     const float* __restrict__ h0, const float* __restrict__ dh_out, float* __restrict__ dh_in,
                     float* __restrict__ daggr, float* __restrict__ dmu, float* __restrict__ dh0_acc,
-                    float* __restrict__ n5_out, float* __restrict__ du_out, float* __restrict__ vec_partial) {
+                    float* __restrict__ n5_out, float* __restrict__ du_out, float* __restrict__ vec_partial,
+                    DropoutArgs drop) {
   using C = NodeBwdCfg<EXTRA>;
   constexpr int DHP = C::DHP, LD = C::LD;
   extern __shared__ __align__(16) float smem[];
@@ -81,20 +85,30 @@ bwd_node_mlp_kernel(int n_nodes, eqd_layer_params p, const float* __restrict__ w
     }
     // ---------------- LeakyReLU + LayerNorm statistics; keep n-hat (smem), sign bits (registers) ----------------
     unsigned pos_lo = 0, pos_hi = 0, pos_x = 0;
+    unsigned keep_lo = 0, keep_hi = 0, keep_x = 0;   // site-2 mask bits, same layout as pos
     const float inv_n = 1.f / (float)p.dh;
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
       float s = 0.f;
+      if (DROPOUT) {   // columns col_nn(tx, 0..7) = 4 tx + 0..3, 32 + 4 tx + 0..3; extra column 64 + tx
+        const unsigned long long key = dropout_key(drop);
+        const unsigned row = (unsigned)(node0 + ty * 8 + i);
+        const unsigned k = dropout_keep4(drop, key, tx, row, drop.c2) | (dropout_keep4(drop, key, 8 + tx, row, drop.c2) << 4);
+        if (i < 4) keep_lo |= k << (i * 8); else keep_hi |= k << ((i - 4) * 8);
+        if (EXTRA) keep_x |= ((dropout_keep4(drop, key, 16 + (tx >> 2), row, drop.c2) >> (tx & 3)) & 1u) << i;
+      }
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
         float a = lrelu(acc[i][j], slope);
         if (a > 0.f) { if (i < 4) pos_lo |= 1u << (i * 8 + j); else pos_hi |= 1u << ((i - 4) * 8 + j); }
+        if (DROPOUT) a *= dropout_mul(i < 4 ? keep_lo : keep_hi, (i & 3) * 8 + j, drop.scale);
         acc[i][j] = a;
         s += a;
       }
       if (EXTRA) {
         float a = xvalid ? lrelu(accx[i], slope) : 0.f;
         if (a > 0.f) pos_x |= 1u << i;
+        if (DROPOUT) a *= dropout_mul(keep_x, i, drop.scale);
         accx[i] = a;
         s += a;
       }
@@ -178,8 +192,10 @@ bwd_node_mlp_kernel(int n_nodes, eqd_layer_params p, const float* __restrict__ w
       for (int j = 0; j < 8; ++j) {
         bool pos = i < 4 ? (pos_lo >> (i * 8 + j)) & 1u : (pos_hi >> ((i - 4) * 8 + j)) & 1u;
         acc[i][j] = rstd * (acc[i][j] - m1 - nhat[j] * m2) * (pos ? 1.f : slope);
+        if (DROPOUT) acc[i][j] *= dropout_mul(i < 4 ? keep_lo : keep_hi, (i & 3) * 8 + j, drop.scale);
       }
       if (EXTRA) accx[i] = xvalid ? rstd * (accx[i] - m1 - nhx * m2) * (((pos_x >> i) & 1u) ? 1.f : slope) : 0.f;
+      if (EXTRA && DROPOUT) accx[i] *= dropout_mul(keep_x, i, drop.scale);
     }
     __syncthreads();   // everyone is done with bufA (A operand of the W6 product)
     store_tile_smem<EXTRA>(bufA, LD, acc, accx, ty, tx);     // du: A operand of the four input-gradient products
@@ -275,11 +291,39 @@ bwd_node_mlp_kernel(int n_nodes, eqd_layer_params p, const float* __restrict__ w
 
 }  // namespace eqd
 
+namespace {
+template <bool EXTRA, bool DROPOUT>
+int launch_bwd_node_mlp(int grid, cudaStream_t st, int n_nodes, const eqd_layer_params& p, const float* w_node1_lin,
+                        const float* w_node2_lin, const float* h_in, int ldh, const float* aggr, const float* mu, int ldmu,
+                        const float* h0, const float* dh_out, float* dh_in, float* daggr, float* dmu, float* dh0_acc,
+                        float* n5_out, float* du_out, float* vec_partial, const eqd::DropoutArgs& d) {
+  size_t smem = eqd::NodeBwdCfg<EXTRA>::SMEM;
+  EQD_SET_SMEM((eqd::bwd_node_mlp_kernel<EXTRA, DROPOUT>), smem);
+  eqd::bwd_node_mlp_kernel<EXTRA, DROPOUT><<<grid, EQD_THREADS, smem, st>>>(n_nodes, p, w_node1_lin, w_node2_lin, h_in, ldh,
+                                                                           aggr, mu, ldmu, h0, dh_out, dh_in, daggr, dmu,
+                                                                           dh0_acc, n5_out, du_out, vec_partial, d);
+  EQD_CUDA_LAUNCH_CHECK();
+  return EQD_OK;
+}
+}  // namespace
+
 extern "C" int eqd_bwd_node_mlp(const eqd_graph* g, const eqd_layer* p_l, const float* w_node1_lin,
                                 const float* w_node2_lin, const float* h_in, int32_t ldh, const float* aggr,
                                 const float* mu, int32_t ldmu, const float* h0, const float* dh_out, float* dh_in,
                                 float* daggr, float* dmu, float* dh0_acc, float* n5_out, float* du_out,
                                 float* vec_partial, int32_t* n_partials_out, void* stream) {
+  return eqd_bwd_node_mlp_dropout(g, p_l, w_node1_lin, w_node2_lin, h_in, ldh, aggr, mu, ldmu, h0, dh_out, dh_in, daggr, dmu,
+                                  dh0_acc, n5_out, du_out, vec_partial, n_partials_out, nullptr, 0, stream);
+}
+
+extern "C" int eqd_bwd_node_mlp_dropout(const eqd_graph* g, const eqd_layer* p_l, const float* w_node1_lin,
+                                        const float* w_node2_lin, const float* h_in, int32_t ldh, const float* aggr,
+                                        const float* mu, int32_t ldmu, const float* h0, const float* dh_out, float* dh_in,
+                                        float* daggr, float* dmu, float* dh0_acc, float* n5_out, float* du_out,
+                                        float* vec_partial, int32_t* n_partials_out, const eqd_dropout* dropout,
+                                        int32_t layer, void* stream) {
+  eqd::DropoutArgs d{};
+  if (const int rc = eqd::dropout_args(dropout, layer, 2, &d)) return rc;
   const eqd_layer_params* p = p_l ? &p_l->dev : nullptr;
   if (!g || !p || !w_node1_lin || !w_node2_lin || !h_in || !aggr || !mu || !h0 || !dh_out || !dh_in || !daggr || !dmu ||
       !dh0_acc || !n5_out || !du_out || !vec_partial)
@@ -293,19 +337,8 @@ extern "C" int eqd_bwd_node_mlp(const eqd_graph* g, const eqd_layer* p_l, const 
   if (n_partials_out) *n_partials_out = grid > 0 ? grid : 0;
   if (g->n_nodes <= 0) return EQD_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  if (extra) {
-    size_t smem = eqd::NodeBwdCfg<true>::SMEM;
-    EQD_SET_SMEM((eqd::bwd_node_mlp_kernel<true>), smem);
-    eqd::bwd_node_mlp_kernel<true><<<grid, EQD_THREADS, smem, st>>>(g->n_nodes, *p, w_node1_lin, w_node2_lin, h_in, ldh, aggr,
-                                                                   mu, ldmu, h0, dh_out, dh_in, daggr, dmu, dh0_acc, n5_out,
-                                                                   du_out, vec_partial);
-  } else {
-    size_t smem = eqd::NodeBwdCfg<false>::SMEM;
-    EQD_SET_SMEM((eqd::bwd_node_mlp_kernel<false>), smem);
-    eqd::bwd_node_mlp_kernel<false><<<grid, EQD_THREADS, smem, st>>>(g->n_nodes, *p, w_node1_lin, w_node2_lin, h_in, ldh,
-                                                                    aggr, mu, ldmu, h0, dh_out, dh_in, daggr, dmu, dh0_acc,
-                                                                    n5_out, du_out, vec_partial);
-  }
-  EQD_CUDA_LAUNCH_CHECK();
-  return EQD_OK;
+  auto launch = extra ? (dropout ? launch_bwd_node_mlp<true, true> : launch_bwd_node_mlp<true, false>)
+                      : (dropout ? launch_bwd_node_mlp<false, true> : launch_bwd_node_mlp<false, false>);
+  return launch(grid, st, g->n_nodes, *p, w_node1_lin, w_node2_lin, h_in, ldh, aggr, mu, ldmu, h0, dh_out, dh_in, daggr, dmu,
+                dh0_acc, n5_out, du_out, vec_partial, d);
 }

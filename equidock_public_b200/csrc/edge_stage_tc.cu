@@ -20,6 +20,7 @@
 // coordinate gathers leave two GEMMs early; the coordinate update runs on threads that do no aggregation) and the fp32
 // epilogue arithmetic is written on lane pairs (add / mul / fma.f32x2: the same IEEE results in half the instructions).
 #include "tc_common.cuh"
+#include "dropout.cuh"
 
 namespace eqd {
 #define TC_THREADS 512
@@ -58,10 +59,14 @@ struct EdgeConsts {                       // per-layer vectors, passed by value 
 // 512 threads = 2 tile groups x 256; in a group, thread (r = q & 127, half = q >> 7) owns columns
 // [32*half, 32*half+32) of edge row r (TMEM lane r): two threads per row keep the per-thread register
 // footprint <= 128 so that 16 warps (4 per scheduler) hide each other's latencies.
+// DROPOUT (training, dropout.cuh): sites 0 (edge_mlp, c2 = drop.c2) and 1 (coors_mlp, c2 + 1).  Each thread generates the keep
+// bits of its 32 columns of a site as ONE 32-bit word right before the epilogue that applies them; mask x scale is applied
+// after the LeakyReLU (positively homogeneous: lrelu(m s z) = m s lrelu(z)).  The p = 0 instantiation is the inference kernel.
+template <bool DROPOUT>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 edge_stage_tc_kernel(eqd_graph g, eqd_layer_params p, const __grid_constant__ EdgeConsts cst,
                      const float* __restrict__ proj, const double* __restrict__ x_in, const double* __restrict__ x_orig,
-                     float* __restrict__ aggr, double* __restrict__ x_out, int* __restrict__ status, int tn) {
+                     float* __restrict__ aggr, double* __restrict__ x_out, int* __restrict__ status, int tn, DropoutArgs drop) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   TcSmem& S = *reinterpret_cast<TcSmem*>(smem_raw);
   const int tid = threadIdx.x, wg = tid >> 8, q = tid & 255, half = q >> 7, r = q & 127, warp = tid >> 5;
@@ -295,6 +300,8 @@ edge_stage_tc_kernel(eqd_graph g, eqd_layer_params p, const __grid_constant__ Ed
           // two IEEE results -- bitwise the scalar sequence, ~5 % fewer instructions in this latency-bound kernel)
         float2 s01 = f2(0.f, 0.f), s23 = f2(0.f, 0.f);
         const float2 sl2 = f2(slope, slope);
+        unsigned keep = 0;
+        if (DROPOUT) keep = dropout_keep32(drop, dropout_key(drop), 8 * half, (unsigned)(e0 + r), drop.c2);
 #pragma unroll
         for (int c4 = 0; c4 < 8; ++c4) {
           float4 a = ps[c4], b = pd[c4];
@@ -302,6 +309,10 @@ edge_stage_tc_kernel(eqd_graph g, eqd_layer_params p, const __grid_constant__ Ed
           float2 x23 = __fadd2_rn(__fadd2_rn(f2(v[c4 * 4 + 2], v[c4 * 4 + 3]), f2(a.z, a.w)), f2(b.z, b.w));
           float2 y01 = __fmul2_rn(x01, sl2), y23 = __fmul2_rn(x23, sl2);
           float2 t01 = f2(fmaxf(x01.x, y01.x), fmaxf(x01.y, y01.y)), t23 = f2(fmaxf(x23.x, y23.x), fmaxf(x23.y, y23.y));
+          if (DROPOUT) {   // site 0: before the LayerNorm statistics
+            t01 = __fmul2_rn(t01, f2(dropout_mul(keep, c4 * 4 + 0, drop.scale), dropout_mul(keep, c4 * 4 + 1, drop.scale)));
+            t23 = __fmul2_rn(t23, f2(dropout_mul(keep, c4 * 4 + 2, drop.scale), dropout_mul(keep, c4 * 4 + 3, drop.scale)));
+          }
           v[c4 * 4 + 0] = t01.x; v[c4 * 4 + 1] = t01.y; v[c4 * 4 + 2] = t23.x; v[c4 * 4 + 3] = t23.y;
           s01 = __fadd2_rn(s01, t01);
           s23 = __fadd2_rn(s23, t23);
@@ -442,13 +453,20 @@ edge_stage_tc_kernel(eqd_graph g, eqd_layer_params p, const __grid_constant__ Ed
       {
         float2 p01 = f2(0.f, 0.f), p23 = f2(0.f, 0.f);
         const float2 sl2 = f2(slope, slope);
+        unsigned keep = 0;
+        if (DROPOUT) keep = dropout_keep32(drop, dropout_key(drop), 8 * half, (unsigned)(e0 + r), drop.c2 + 1);
 #pragma unroll
         for (int c = 0; c < 32; c += 4) {
           float2 x01 = __fadd2_rn(f2(v[c], v[c + 1]), f2(cst.b3[half * 32 + c], cst.b3[half * 32 + c + 1]));
           float2 x23 = __fadd2_rn(f2(v[c + 2], v[c + 3]), f2(cst.b3[half * 32 + c + 2], cst.b3[half * 32 + c + 3]));
           float2 y01 = __fmul2_rn(x01, sl2), y23 = __fmul2_rn(x23, sl2);
-          p01 = __ffma2_rn(f2(fmaxf(x01.x, y01.x), fmaxf(x01.y, y01.y)), f2(cst.w4[half * 32 + c], cst.w4[half * 32 + c + 1]), p01);
-          p23 = __ffma2_rn(f2(fmaxf(x23.x, y23.x), fmaxf(x23.y, y23.y)), f2(cst.w4[half * 32 + c + 2], cst.w4[half * 32 + c + 3]), p23);
+          float2 t01 = f2(fmaxf(x01.x, y01.x), fmaxf(x01.y, y01.y)), t23 = f2(fmaxf(x23.x, y23.x), fmaxf(x23.y, y23.y));
+          if (DROPOUT) {   // site 1: lrelu(z3) before the w4 dot product
+            t01 = __fmul2_rn(t01, f2(dropout_mul(keep, c + 0, drop.scale), dropout_mul(keep, c + 1, drop.scale)));
+            t23 = __fmul2_rn(t23, f2(dropout_mul(keep, c + 2, drop.scale), dropout_mul(keep, c + 3, drop.scale)));
+          }
+          p01 = __ffma2_rn(t01, f2(cst.w4[half * 32 + c], cst.w4[half * 32 + c + 1]), p01);
+          p23 = __ffma2_rn(t23, f2(cst.w4[half * 32 + c + 2], cst.w4[half * 32 + c + 3]), p23);
         }
         ph4[0] = p01.x; ph4[1] = p01.y; ph4[2] = p23.x; ph4[3] = p23.y;
       }
@@ -500,8 +518,9 @@ edge_stage_tc_kernel(eqd_graph g, eqd_layer_params p, const __grid_constant__ Ed
 
 EQD_TRACE_SETTER(eqd_trace_set_edge)
 
-extern "C" int eqd_edge_stage(const eqd_graph* g, const eqd_layer* p_l, const float* proj, const double* x_in,
-                              const double* x_orig, float* aggr, double* x_out, int32_t* status, void* stream) {
+namespace eqd {
+int edge_stage_tc(const eqd_graph* g, const eqd_layer* p_l, const float* proj, const double* x_in, const double* x_orig,
+                  float* aggr, double* x_out, int32_t* status, const DropoutArgs* drop, void* stream) {
   const eqd_layer_params* p = p_l ? &p_l->dev : nullptr;
   if (!g || !p || !proj || !x_in || !x_orig || !aggr || !x_out || !status) return EQD_ERR_BAD_ARG;
   if (!p->w_edge_tc) return EQD_ERR_BAD_ARG;
@@ -514,14 +533,26 @@ extern "C" int eqd_edge_stage(const eqd_graph* g, const eqd_layer* p_l, const fl
   int tn = EQD_TM / g->max_in_degree;
   if (tn > TC_MAX_TN) tn = TC_MAX_TN;
   int ntiles = (g->n_nodes + tn - 1) / tn;
-  eqd::EdgeConsts cst;
+  EdgeConsts cst;
   memcpy(&cst, p_l->consts.edge, sizeof(cst));
-  size_t smem = sizeof(eqd::TcSmem) + 128;
-  EQD_SET_SMEM((eqd::edge_stage_tc_kernel), smem);
+  size_t smem = sizeof(TcSmem) + 128;
   int grid = (ntiles + 1) / 2;
   if (grid > 148) grid = 148;
-  eqd::edge_stage_tc_kernel<<<grid, TC_THREADS, smem, (cudaStream_t)stream>>>(*g, *p, cst, proj, x_in, x_orig, aggr, x_out,
-                                                                             status, tn);
+  if (drop) {
+    EQD_SET_SMEM((eqd::edge_stage_tc_kernel<true>), smem);
+    eqd::edge_stage_tc_kernel<true><<<grid, TC_THREADS, smem, (cudaStream_t)stream>>>(*g, *p, cst, proj, x_in, x_orig, aggr,
+                                                                                     x_out, status, tn, *drop);
+  } else {
+    EQD_SET_SMEM((eqd::edge_stage_tc_kernel<false>), smem);
+    eqd::edge_stage_tc_kernel<false><<<grid, TC_THREADS, smem, (cudaStream_t)stream>>>(*g, *p, cst, proj, x_in, x_orig, aggr,
+                                                                                      x_out, status, tn, DropoutArgs{});
+  }
   EQD_CUDA_LAUNCH_CHECK();
   return EQD_OK;
+}
+}  // namespace eqd
+
+extern "C" int eqd_edge_stage(const eqd_graph* g, const eqd_layer* p_l, const float* proj, const double* x_in,
+                              const double* x_orig, float* aggr, double* x_out, int32_t* status, void* stream) {
+  return eqd::edge_stage_tc(g, p_l, proj, x_in, x_orig, aggr, x_out, status, nullptr, stream);
 }

@@ -7,6 +7,7 @@
 #include <cstring>
 
 #include "common.cuh"
+#include "dropout.cuh"
 
 namespace {
 
@@ -84,7 +85,17 @@ extern "C" int eqd_forward_stash_offsets(const eqd_graph* g, int32_t n_layers, s
 extern "C" int eqd_iegmn_forward(const eqd_graph* g, const eqd_layer* const* layers, int32_t n_layers,
                                  const eqd_head_params* hp, const eqd_forward_io* io, void* workspace,
                                  size_t workspace_bytes, void* stream) {
+  return eqd_iegmn_forward_dropout(g, layers, n_layers, hp, io, nullptr, workspace, workspace_bytes, stream);
+}
+
+extern "C" int eqd_iegmn_forward_dropout(const eqd_graph* g, const eqd_layer* const* layers, int32_t n_layers,
+                                         const eqd_head_params* hp, const eqd_forward_io* io, const eqd_dropout* dropout,
+                                         void* workspace, size_t workspace_bytes, void* stream) {
   if (!g || !layers || n_layers < 1 || !hp || !io || !workspace) return EQD_ERR_BAD_ARG;
+  // per-site kernel arguments: drop[li][0] = the edge stage's (sites 0, 1), drop[li][1] = node_mlp's (site 2); head: site 3
+  eqd::DropoutArgs dhead{};
+  if (int rc = eqd::dropout_args(dropout, n_layers, 3, &dhead)) return rc;
+  if (dropout && io->layer0_fp32) return EQD_ERR_UNSUPPORTED;   // the fp32 CUDA-core twins have no dropout
   if (!io->emb || !io->res_lig || !io->res_rec || !io->mu_lig || !io->mu_rec || !io->x_lig || !io->x_rec || !io->rot ||
       !io->trans || !io->ligand_out || !io->sing || !io->status || !io->h_out || !io->x_out)
     return EQD_ERR_BAD_ARG;
@@ -166,15 +177,22 @@ extern "C" int eqd_iegmn_forward(const eqd_graph* g, const eqd_layer* const* lay
       aggr = reinterpret_cast<float*>(sb + sl.aggr + (size_t)li * sl.a_stride);
       mu = reinterpret_cast<float*>(sb + sl.mu + (size_t)li * sl.m_stride);
     }
+    eqd::DropoutArgs de{}, dn{};
+    if (dropout) {
+      eqd::dropout_args(dropout, li, 0, &de);
+      eqd::dropout_args(dropout, li, 2, &dn);
+    }
     stage_event(li, 0);
-    rc = eqd_edge_stage(g, lp_l, pa, x_in, x0, aggr, x_out, io->status, stream);
+    rc = eqd::edge_stage_tc(g, lp_l, pa, x_in, x0, aggr, x_out, io->status, dropout ? &de : nullptr, stream);
     if (rc) return rc;
     stage_event(li, 1);
     stage_event(li, 2);
     if (lp->dh == EQD_HID && lp->w_node_tc && (!lpn || lpn->w_proj_tc)) {
-      rc = eqd_node_stage_tc(g, lp_l, lpn_l, h_in, h0, pa, aggr, kv, mu, h_out, pb, stream);
+      rc = eqd::node_stage_tc(g, lp_l, lpn_l, h_in, h0, pa, aggr, kv, mu, h_out, pb, dropout ? &dn : nullptr, stream);
     } else if (li == 0 && tc0 && (!lpn || lpn->w_proj_tc)) {
-      rc = eqd_node_stage_tc0(g, lp_l, lpn_l, h0, pa, aggr, kv, x5, mu, h_out, pb, stream);
+      rc = eqd::node_stage_tc0(g, lp_l, lpn_l, h0, pa, aggr, kv, x5, mu, h_out, pb, dropout ? &dn : nullptr, stream);
+    } else if (dropout) {
+      return EQD_ERR_UNSUPPORTED;
     } else {   // fp32 CUDA-core node stage (fused projections); the next layer's tensor-core attention needs K/V blocks
       rc = eqd_node_stage(g, lp_l, lpn_l, h_in, ldh, h0, pa, aggr, h_out, pb, stream);
       if (!rc && lpn && lpn->dh == EQD_HID && lpn->w_node_tc) rc = eqd_kv_blocks(g, pb, 320, 192, 256, kv, stream);
@@ -189,9 +207,33 @@ extern "C" int eqd_iegmn_forward(const eqd_graph* g, const eqd_layer* const* lay
     x_in = x_out;
   }
   if (dbg & 1) return EQD_OK;
-  rc = eqd_keypoints(g, hp, h_in, x_in, w + c.head, c.head_bytes, keypts, ymean, cov, stream);
+  rc = eqd::keypoints(g, hp, h_in, x_in, w + c.head, c.head_bytes, keypts, ymean, cov, dropout ? &dhead : nullptr, stream);
   if (rc) return rc;
   return eqd_kabsch_apply(g, cov, ymean, io->x_lig, nullptr, io->rot, io->trans, io->ligand_out, io->sing, io->status, stream);
+}
+
+// ---- dropout keep masks for tests and oracles (dropout.cuh) --------------------------------------------------------------
+namespace eqd {
+__global__ void dropout_mask_kernel(DropoutArgs d, int rows, int cols, unsigned char* __restrict__ keep) {
+  const int nc4 = (cols + 3) / 4;
+  const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (long)rows * nc4) return;
+  const int r = (int)(i / nc4), c4 = (int)(i - (long)r * nc4);
+  const unsigned bits = dropout_keep4(d, dropout_key(d), (unsigned)c4, (unsigned)r, d.c2);
+  for (int j = 0; j < 4 && c4 * 4 + j < cols; ++j) keep[(long)r * cols + c4 * 4 + j] = (bits >> j) & 1u;
+}
+}  // namespace eqd
+
+extern "C" int eqd_dropout_mask(const eqd_dropout* dropout, int32_t layer, int32_t site, int32_t rows, int32_t cols,
+                                uint8_t* keep, void* stream) {
+  if (!dropout || !keep || rows < 0 || cols < 0) return EQD_ERR_BAD_ARG;
+  eqd::DropoutArgs d{};
+  if (int rc = eqd::dropout_args(dropout, layer, site, &d)) return rc;
+  const long n = (long)rows * ((cols + 3) / 4);
+  if (n == 0) return EQD_OK;
+  eqd::dropout_mask_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(d, rows, cols, keep);
+  EQD_CUDA_LAUNCH_CHECK();
+  return EQD_OK;
 }
 
 // Thin CUDA event helpers so that a binding without its own CUDA runtime access can time the stages of

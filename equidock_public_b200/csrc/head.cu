@@ -11,6 +11,7 @@
 
 #include "common.cuh"
 #include "svd3.cuh"
+#include "dropout.cuh"
 
 namespace eqd {
 
@@ -20,8 +21,10 @@ namespace eqd {
 #define HEAD_JC 64    // nodes per staged chunk
 
 // ---- partial column sums of LeakyReLU(W_m h + b_m) over each node tile (:525, :529) -------------
+// DROPOUT (training, dropout.cuh): site 3 (mlp_h_mean_ROT, c2 = drop.c2), mask x scale before the column sums.
+template <bool DROPOUT>
 __global__ void __launch_bounds__(EQD_THREADS, 2)
-head_mean_kernel(eqd_graph g, eqd_head_params hp, const float* __restrict__ h, float* __restrict__ part) {
+head_mean_kernel(eqd_graph g, eqd_head_params hp, const float* __restrict__ h, float* __restrict__ part, DropoutArgs drop) {
   TRACE_START(5);
   extern __shared__ __align__(16) float smem[];
   constexpr int LD = 68;
@@ -44,8 +47,18 @@ head_mean_kernel(eqd_graph g, eqd_head_params hp, const float* __restrict__ h, f
 #pragma unroll
     for (int i = 0; i < 8; ++i)
       if (ty * 8 + i < nvalid) {
+        unsigned keep = 0;
+        if (DROPOUT) {   // columns 4 tx .. 4 tx + 3 and 32 + 4 tx .. 32 + 4 tx + 3 (col_nn)
+          const unsigned long long key = dropout_key(drop);
+          const unsigned row = (unsigned)(node0 + ty * 8 + i);
+          keep = dropout_keep4(drop, key, tx, row, drop.c2) | (dropout_keep4(drop, key, 8 + tx, row, drop.c2) << 4);
+        }
 #pragma unroll
-        for (int j = 0; j < 8; ++j) colsum[j] += lrelu(acc[i][j], hp.leaky_slope);
+        for (int j = 0; j < 8; ++j) {
+          float a = lrelu(acc[i][j], hp.leaky_slope);
+          if (DROPOUT) a *= dropout_mul(keep, j, drop.scale);
+          colsum[j] += a;
+        }
       }
 #pragma unroll
     for (int j = 0; j < 8; ++j) wbuf[ty * 64 + col_nn(tx, j)] = colsum[j];
@@ -385,9 +398,9 @@ extern "C" int eqd_head_fold(const eqd_head_params* hp, double* m_qk, void* stre
   return EQD_OK;
 }
 
-extern "C" int eqd_keypoints(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x,
-                             void* workspace, size_t workspace_bytes, double* keypts, double* ymean, double* cov,
-                             void* stream) {
+namespace eqd {
+int keypoints(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x, void* workspace,
+              size_t workspace_bytes, double* keypts, double* ymean, double* cov, const DropoutArgs* drop, void* stream) {
   if (!g || !hp || !h || !x || !workspace || !keypts || !ymean || !cov) return EQD_ERR_BAD_ARG;
   if (!hp->m_qk || (reinterpret_cast<uintptr_t>(hp->m_qk) & 15)) return EQD_ERR_BAD_ARG;   // eqd_head_fold() output
   if (workspace_bytes < eqd_workspace_bytes(g->n_nodes, g->n_node_tiles, g->n_pairs)) return EQD_ERR_WORKSPACE;
@@ -402,9 +415,14 @@ extern "C" int eqd_keypoints(const eqd_graph* g, const eqd_head_params* hp, cons
   const int nseg = 2 * g->n_pairs;
   {
     size_t smem = (size_t)(EQD_TM * 68 + 2 * EQD_WCHUNK * EQD_WLD) * sizeof(float);
-    EQD_SET_SMEM((eqd::head_mean_kernel), smem);
     int grid = g->n_node_tiles < 148 * 2 ? g->n_node_tiles : 148 * 2;
-    eqd::head_mean_kernel<<<grid, EQD_THREADS, smem, st>>>(*g, *hp, h, part);
+    if (drop) {
+      EQD_SET_SMEM((eqd::head_mean_kernel<true>), smem);
+      eqd::head_mean_kernel<true><<<grid, EQD_THREADS, smem, st>>>(*g, *hp, h, part, *drop);
+    } else {
+      EQD_SET_SMEM((eqd::head_mean_kernel<false>), smem);
+      eqd::head_mean_kernel<false><<<grid, EQD_THREADS, smem, st>>>(*g, *hp, h, part, DropoutArgs{});
+    }
     EQD_CUDA_LAUNCH_CHECK();
   }
   {
@@ -430,6 +448,13 @@ extern "C" int eqd_keypoints(const eqd_graph* g, const eqd_head_params* hp, cons
     EQD_CUDA_LAUNCH_CHECK();
   }
   return EQD_OK;
+}
+}  // namespace eqd
+
+extern "C" int eqd_keypoints(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x,
+                             void* workspace, size_t workspace_bytes, double* keypts, double* ymean, double* cov,
+                             void* stream) {
+  return eqd::keypoints(g, hp, h, x, workspace, workspace_bytes, keypts, ymean, cov, nullptr, stream);
 }
 
 extern "C" int eqd_kabsch_apply(const eqd_graph* g, const double* cov, const double* ymean, const float* x_lig_in,
@@ -729,11 +754,12 @@ __global__ void head_dqbar_kernel(int n_pairs, eqd_head_params hp, const double*
   dqbar[(long)p * 64 + dq] = t;
 }
 
-// warp per node: pre = W_m h + b_m; dpre = dqbar[seg] / n_seg * lrelu'(pre) -> dpre_out (D operand of dW_m);
-// dh[n] += W_m^T dpre
+// warp per node: pre = W_m h + b_m; dpre = dqbar[seg] / n_seg * lrelu'(pre) (* the site-3 dropout multiplier) -> dpre_out
+// (D operand of dW_m); dh[n] += W_m^T dpre
+template <bool DROPOUT>
 __global__ void head_mean_bwd_kernel(eqd_graph g, eqd_head_params hp, const int* __restrict__ node_seg,
                                      const float* __restrict__ h, const double* __restrict__ dqbar,
-                                     float* __restrict__ dpre_out, float* __restrict__ dh) {
+                                     float* __restrict__ dpre_out, float* __restrict__ dh, DropoutArgs drop) {
   __shared__ float hs[8][64], dp[8][64];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n = blockIdx.x * 8 + w;
@@ -748,8 +774,13 @@ __global__ void head_mean_bwd_kernel(eqd_graph g, eqd_head_params hp, const int*
     p0 = fmaf(hs[w][d], hp.w_mean[d * 64 + lane], p0);
     p1 = fmaf(hs[w][d], hp.w_mean[d * 64 + lane + 32], p1);
   }
-  const float g0 = (float)dqbar[(long)s * 64 + lane] * inv_n * (p0 > 0.f ? 1.f : hp.leaky_slope);
-  const float g1 = (float)dqbar[(long)s * 64 + lane + 32] * inv_n * (p1 > 0.f ? 1.f : hp.leaky_slope);
+  float g0 = (float)dqbar[(long)s * 64 + lane] * inv_n * (p0 > 0.f ? 1.f : hp.leaky_slope);
+  float g1 = (float)dqbar[(long)s * 64 + lane + 32] * inv_n * (p1 > 0.f ? 1.f : hp.leaky_slope);
+  if (DROPOUT) {   // columns lane and lane + 32: words lane % 4 of counters lane / 4 and 8 + lane / 4
+    const unsigned long long key = dropout_key(drop);
+    g0 *= dropout_mul(dropout_keep4(drop, key, lane >> 2, (unsigned)n, drop.c2), lane & 3, drop.scale);
+    g1 *= dropout_mul(dropout_keep4(drop, key, 8 + (lane >> 2), (unsigned)n, drop.c2), lane & 3, drop.scale);
+  }
   dpre_out[(long)n * 64 + lane] = g0;
   dpre_out[(long)n * 64 + lane + 32] = g1;
   dp[w][lane] = g0;
@@ -784,10 +815,11 @@ extern "C" size_t eqd_bwd_head_workspace_bytes(int32_t n_nodes, int32_t n_node_t
 // may be NULL), drot [B][9], dtrans [B][3] (fp32, may be NULL).  Outputs: dh [n][64] (fp32, overwritten), dx [n][3]
 // (fp64, overwritten), dpre [n][64] (the D operand of d mlp_h_mean_ROT.0.weight = dpre^T h, reduced by the caller with
 // eqd_tn_gemm), and the head weight gradients accumulated into g_wkey / g_wquery (state_dict layouts [3200][64]).
-extern "C" int eqd_bwd_head(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x,
-                            const double* cov, const float* x_lig_in, const float* dcoors, const double* dkeypts,
-                            const float* drot, const float* dtrans, void* workspace, size_t workspace_bytes, float* dh,
-                            double* dx, float* dpre, float* g_wkey, float* g_wquery, void* stream) {
+namespace eqd {
+static int bwd_head(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x, const double* cov,
+                    const float* x_lig_in, const float* dcoors, const double* dkeypts, const float* drot, const float* dtrans,
+                    void* workspace, size_t workspace_bytes, float* dh, double* dx, float* dpre, float* g_wkey,
+                    float* g_wquery, const DropoutArgs* drop, void* stream) {
   if (!g || !hp || !h || !x || !cov || !x_lig_in || !workspace || !dh || !dx || !dpre || !g_wkey || !g_wquery)
     return EQD_ERR_BAD_ARG;
   if (workspace_bytes < eqd_bwd_head_workspace_bytes(g->n_nodes, g->n_node_tiles, g->n_pairs)) return EQD_ERR_WORKSPACE;
@@ -810,7 +842,7 @@ extern "C" int eqd_bwd_head(const eqd_graph* g, const eqd_head_params* hp, const
   double* a = reinterpret_cast<double*>(take(2 * B * EQD_HEADS * 64 * 8));
   double* dqbar = reinterpret_cast<double*>(take(2 * B * 64 * 8));
   // recompute qbar, u, keypoints and their means (cov_scratch is discarded: the caller's cov may carry the guard's noise)
-  int rc = eqd_keypoints(g, hp, h, x, fwd_ws, fwd_bytes, keypts, ymean, cov_scratch, stream);
+  int rc = keypoints(g, hp, h, x, fwd_ws, fwd_bytes, keypts, ymean, cov_scratch, drop, stream);
   if (rc) return rc;
   const double* qbar = reinterpret_cast<const double*>(fwd_ws + ws_part_bytes(g->n_node_tiles) + ws_tile_ptr_bytes(g->n_pairs));
   const double* u = reinterpret_cast<const double*>(reinterpret_cast<const unsigned char*>(qbar) + ws_qbar_bytes(g->n_pairs));
@@ -830,9 +862,34 @@ extern "C" int eqd_bwd_head(const eqd_graph* g, const eqd_head_params* hp, const
   EQD_CUDA_LAUNCH_CHECK();
   eqd::head_dqbar_kernel<<<2 * g->n_pairs, 64, 0, st>>>(g->n_pairs, *hp, a, dqbar);
   EQD_CUDA_LAUNCH_CHECK();
-  eqd::head_mean_bwd_kernel<<<(unsigned)((N + 7) / 8), 256, 0, st>>>(*g, *hp, node_seg, h, dqbar, dpre, dh);
+  if (drop)
+    eqd::head_mean_bwd_kernel<true><<<(unsigned)((N + 7) / 8), 256, 0, st>>>(*g, *hp, node_seg, h, dqbar, dpre, dh, *drop);
+  else
+    eqd::head_mean_bwd_kernel<false><<<(unsigned)((N + 7) / 8), 256, 0, st>>>(*g, *hp, node_seg, h, dqbar, dpre, dh,
+                                                                             DropoutArgs{});
   EQD_CUDA_LAUNCH_CHECK();
   return EQD_OK;
+}
+}  // namespace eqd
+
+extern "C" int eqd_bwd_head(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x,
+                            const double* cov, const float* x_lig_in, const float* dcoors, const double* dkeypts,
+                            const float* drot, const float* dtrans, void* workspace, size_t workspace_bytes, float* dh,
+                            double* dx, float* dpre, float* g_wkey, float* g_wquery, void* stream) {
+  return eqd::bwd_head(g, hp, h, x, cov, x_lig_in, dcoors, dkeypts, drot, dtrans, workspace, workspace_bytes, dh, dx, dpre,
+                       g_wkey, g_wquery, nullptr, stream);
+}
+
+extern "C" int eqd_bwd_head_dropout(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x,
+                                    const double* cov, const float* x_lig_in, const float* dcoors, const double* dkeypts,
+                                    const float* drot, const float* dtrans, void* workspace, size_t workspace_bytes,
+                                    float* dh, double* dx, float* dpre, float* g_wkey, float* g_wquery,
+                                    const eqd_dropout* dropout, int32_t layer, void* stream) {
+  eqd::DropoutArgs d;
+  const int rc = eqd::dropout_args(dropout, layer, 3, &d);
+  if (rc) return rc;
+  return eqd::bwd_head(g, hp, h, x, cov, x_lig_in, dcoors, dkeypts, drot, dtrans, workspace, workspace_bytes, dh, dx, dpre,
+                       g_wkey, g_wquery, dropout ? &d : nullptr, stream);
 }
 
 // =====================================================================================================================

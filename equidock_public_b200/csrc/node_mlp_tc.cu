@@ -3,6 +3,7 @@
 // Weight-stationary (W5: 64x272, W6: 64x64 as bf16x3 UMMA panels, 126 KB in shared memory), two tile groups of
 // 256 threads (2 threads per node row) running out of phase.  The 272-wide input is fed in 5 K-pieces.
 #include "tc_common.cuh"
+#include "dropout.cuh"
 
 namespace eqd {
 
@@ -24,10 +25,13 @@ struct NmSmem {
   unsigned int tmem_base;
 };
 
+// DROPOUT (training, dropout.cuh): site 2 (node_mlp, c2 = drop.c2), mask x scale after the LeakyReLU of u5, before the
+// LayerNorm statistics; 8 Philox calls per thread give the keep bits of its 32 columns.
+template <bool DROPOUT>
 __global__ void __launch_bounds__(NM_THREADS, 1)
 node_mlp_tc_kernel(int n_nodes, eqd_layer_params p, const __grid_constant__ NmConsts cst, const float* __restrict__ h_in,
                    const float* __restrict__ aggr, const float* __restrict__ mu, const float* __restrict__ h0,
-                   float* __restrict__ h_out) {
+                   float* __restrict__ h_out, DropoutArgs drop) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   NmSmem& S = *reinterpret_cast<NmSmem*>(smem_raw);
   const int tid = threadIdx.x, wg = tid >> 8, q = tid & 255, half = q >> 7, r = q & 127, warp = tid >> 5;
@@ -177,9 +181,12 @@ node_mlp_tc_kernel(int n_nodes, eqd_layer_params p, const __grid_constant__ NmCo
     {
       float v[32];
       float s4[4] = {0.f, 0.f, 0.f, 0.f};
+      unsigned keep = 0;
+      if (DROPOUT) keep = dropout_keep32(drop, dropout_key(drop), 8 * half, (unsigned)node, drop.c2);
 #pragma unroll
       for (int c = 0; c < 32; ++c) {
         v[c] = lrelu(acc[c], slope);
+        if (DROPOUT) v[c] *= dropout_mul(keep, c, drop.scale);
         s4[c & 3] += v[c];
       }
       const float mh = ((s4[0] + s4[1]) + (s4[2] + s4[3])) * (1.f / 32.f);
@@ -258,9 +265,12 @@ struct Nm0Smem {
   unsigned int tmem_base;
 };
 
+// DROPOUT: site 2 as above, on the 69 real channels (half 0 also masks the extra columns 64..68).
+template <bool DROPOUT>
 __global__ void __launch_bounds__(NM_THREADS, 1)
 node_mlp0_tc_kernel(int n_nodes, eqd_layer_params p, const __grid_constant__ Nm0Consts cst, const float* __restrict__ h0,
-                    const float* __restrict__ aggr, const float* __restrict__ mu /*[n][72]*/, float* __restrict__ h_out) {
+                    const float* __restrict__ aggr, const float* __restrict__ mu /*[n][72]*/, float* __restrict__ h_out,
+                    DropoutArgs drop) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   Nm0Smem& S = *reinterpret_cast<Nm0Smem*>(smem_raw);
   const int tid = threadIdx.x, wg = tid >> 8, q = tid & 255, half = q >> 7, r = q & 127, warp = tid >> 5;
@@ -393,15 +403,23 @@ node_mlp0_tc_kernel(int n_nodes, eqd_layer_params p, const __grid_constant__ Nm0
     {
       const int nh = half == 0 ? 37 : 32;
       float sum = 0.f;
+      unsigned keep = 0, keepx = 0;
+      if (DROPOUT) {
+        const unsigned long long key = dropout_key(drop);
+        keep = dropout_keep32(drop, key, 8 * half, (unsigned)node, drop.c2);
+        if (half == 0) keepx = dropout_keep4(drop, key, 16, (unsigned)node, drop.c2) | (dropout_keep4(drop, key, 17, (unsigned)node, drop.c2) << 4);
+      }
 #pragma unroll
       for (int c = 0; c < 32; ++c) {
         acc[c] = lrelu(acc[c], slope);
+        if (DROPOUT) acc[c] *= dropout_mul(keep, c, drop.scale);
         sum += acc[c];
       }
       if (half == 0) {
 #pragma unroll
         for (int c = 0; c < 5; ++c) {
           accx[c] = lrelu(accx[c], slope);
+          if (DROPOUT) accx[c] *= dropout_mul(keepx, c, drop.scale);
           sum += accx[c];
         }
       }
@@ -482,78 +500,119 @@ node_mlp0_tc_kernel(int n_nodes, eqd_layer_params p, const __grid_constant__ Nm0
 
 EQD_TRACE_SETTER(eqd_trace_set_mlp)
 
-extern "C" int eqd_node_mlp_tc(const eqd_graph* g, const eqd_layer* p_l, const float* h_in, const float* aggr,
-                               const float* mu, const float* h0, float* h_out, void* stream) {
+namespace eqd {
+int node_mlp_tc(const eqd_graph* g, const eqd_layer* p_l, const float* h_in, const float* aggr, const float* mu,
+                const float* h0, float* h_out, const DropoutArgs* drop, void* stream) {
   const eqd_layer_params* p = p_l ? &p_l->dev : nullptr;
   if (!g || !p || !h_in || !aggr || !mu || !h0 || !h_out) return EQD_ERR_BAD_ARG;
   if (p->dh != 64 || p->dhp != 64) return EQD_ERR_UNSUPPORTED;
   if (!(p->leaky_slope >= 0.f && p->leaky_slope <= 1.f)) return EQD_ERR_UNSUPPORTED;  // lrelu() = max(v, slope*v)
   if (!p->w_node_tc || (reinterpret_cast<uintptr_t>(p->w_node_tc) & 15)) return EQD_ERR_BAD_ARG;
   if (g->n_nodes <= 0) return EQD_OK;
-  eqd::NmConsts cst;
+  NmConsts cst;
   memcpy(&cst, p_l->consts.node, sizeof(cst));
   int ntiles = (g->n_nodes + EQD_TM - 1) / EQD_TM;
-  size_t smem = sizeof(eqd::NmSmem) + 128;
-  EQD_SET_SMEM((eqd::node_mlp_tc_kernel), smem);
+  size_t smem = sizeof(NmSmem) + 128;
   int grid = (ntiles + 1) / 2;
   if (grid > 148) grid = 148;
-  eqd::node_mlp_tc_kernel<<<grid, NM_THREADS, smem, (cudaStream_t)stream>>>(g->n_nodes, *p, cst, h_in, aggr, mu, h0, h_out);
+  if (drop) {
+    EQD_SET_SMEM((node_mlp_tc_kernel<true>), smem);
+    node_mlp_tc_kernel<true><<<grid, NM_THREADS, smem, (cudaStream_t)stream>>>(g->n_nodes, *p, cst, h_in, aggr, mu, h0, h_out,
+                                                                              *drop);
+  } else {
+    EQD_SET_SMEM((node_mlp_tc_kernel<false>), smem);
+    node_mlp_tc_kernel<false><<<grid, NM_THREADS, smem, (cudaStream_t)stream>>>(g->n_nodes, *p, cst, h_in, aggr, mu, h0, h_out,
+                                                                               DropoutArgs{});
+  }
   EQD_CUDA_LAUNCH_CHECK();
   return EQD_OK;
 }
 
-extern "C" int eqd_node_mlp_tc0(const eqd_graph* g, const eqd_layer* p_l, const float* h0, const float* aggr,
-                                const float* mu, float* h_out, void* stream) {
+int node_mlp_tc0(const eqd_graph* g, const eqd_layer* p_l, const float* h0, const float* aggr, const float* mu,
+                 float* h_out, const DropoutArgs* drop, void* stream) {
   const eqd_layer_params* p = p_l ? &p_l->dev : nullptr;
   if (!g || !p || !h0 || !aggr || !mu || !h_out) return EQD_ERR_BAD_ARG;
   if (p->dh != 69 || p->dhp != 72) return EQD_ERR_UNSUPPORTED;
   if (!(p->leaky_slope >= 0.f && p->leaky_slope <= 1.f)) return EQD_ERR_UNSUPPORTED;  // lrelu() = max(v, slope*v)
   if (!p->w_node_tc || (reinterpret_cast<uintptr_t>(p->w_node_tc) & 15)) return EQD_ERR_BAD_ARG;
   if (g->n_nodes <= 0) return EQD_OK;
-  eqd::Nm0Consts cst;
+  Nm0Consts cst;
   memcpy(&cst, p_l->consts.node, sizeof(cst));
   int ntiles = (g->n_nodes + EQD_TM - 1) / EQD_TM;
-  size_t smem = sizeof(eqd::Nm0Smem) + 128;
-  EQD_SET_SMEM((eqd::node_mlp0_tc_kernel), smem);
+  size_t smem = sizeof(Nm0Smem) + 128;
   int grid = (ntiles + 1) / 2;
   if (grid > 148) grid = 148;
-  eqd::node_mlp0_tc_kernel<<<grid, NM_THREADS, smem, (cudaStream_t)stream>>>(g->n_nodes, *p, cst, h0, aggr, mu, h_out);
+  if (drop) {
+    EQD_SET_SMEM((node_mlp0_tc_kernel<true>), smem);
+    node_mlp0_tc_kernel<true><<<grid, NM_THREADS, smem, (cudaStream_t)stream>>>(g->n_nodes, *p, cst, h0, aggr, mu, h_out, *drop);
+  } else {
+    EQD_SET_SMEM((node_mlp0_tc_kernel<false>), smem);
+    node_mlp0_tc_kernel<false><<<grid, NM_THREADS, smem, (cudaStream_t)stream>>>(g->n_nodes, *p, cst, h0, aggr, mu, h_out,
+                                                                                DropoutArgs{});
+  }
   EQD_CUDA_LAUNCH_CHECK();
   return EQD_OK;
+}
+}  // namespace eqd
+
+extern "C" int eqd_node_mlp_tc(const eqd_graph* g, const eqd_layer* p_l, const float* h_in, const float* aggr,
+                               const float* mu, const float* h0, float* h_out, void* stream) {
+  return eqd::node_mlp_tc(g, p_l, h_in, aggr, mu, h0, h_out, nullptr, stream);
+}
+
+extern "C" int eqd_node_mlp_tc0(const eqd_graph* g, const eqd_layer* p_l, const float* h0, const float* aggr,
+                                const float* mu, float* h_out, void* stream) {
+  return eqd::node_mlp_tc0(g, p_l, h0, aggr, mu, h_out, nullptr, stream);
 }
 
 extern "C" int eqd_attention_tc0(const eqd_graph*, const float*, const void*, const float*, float*, void*);
 
 // Layer 0 (dh == 69): attention (64 tensor-core channels + 5 fp32 ones), node MLP, next layer's projections.
-extern "C" int eqd_node_stage_tc0(const eqd_graph* g, const eqd_layer* p_l, const eqd_layer* p_next_l,
-                                  const float* h0, const float* proj, const float* aggr, void* kv, const float* x5,
-                                  float* mu, float* h_out, float* proj_next, void* stream) {
+namespace eqd {
+int node_stage_tc0(const eqd_graph* g, const eqd_layer* p_l, const eqd_layer* p_next_l, const float* h0, const float* proj,
+                   const float* aggr, void* kv, const float* x5, float* mu, float* h_out, float* proj_next,
+                   const DropoutArgs* drop, void* stream) {
   const eqd_layer_params* p = p_l ? &p_l->dev : nullptr;
   const eqd_layer_params* p_next = p_next_l ? &p_next_l->dev : nullptr;
   if (!g || !p || !kv || !mu || !x5) return EQD_ERR_BAD_ARG;
   if (p_next && !proj_next) return EQD_ERR_BAD_ARG;
   int rc = eqd_attention_tc0(g, proj, kv, x5, mu, stream);
   if (rc) return rc;
-  rc = eqd_node_mlp_tc0(g, p_l, h0, aggr, mu, h_out, stream);
+  rc = node_mlp_tc0(g, p_l, h0, aggr, mu, h_out, drop, stream);
   if (rc) return rc;
   if (p_next) rc = eqd_project_tc(g, p_next_l, h_out, proj_next, kv, stream);
   return rc;
+}
+}  // namespace eqd
+
+extern "C" int eqd_node_stage_tc0(const eqd_graph* g, const eqd_layer* p_l, const eqd_layer* p_next_l,
+                                  const float* h0, const float* proj, const float* aggr, void* kv, const float* x5,
+                                  float* mu, float* h_out, float* proj_next, void* stream) {
+  return eqd::node_stage_tc0(g, p_l, p_next_l, h0, proj, aggr, kv, x5, mu, h_out, proj_next, nullptr, stream);
 }
 
 extern "C" int eqd_project_tc(const eqd_graph*, const eqd_layer*, const float*, float*, void*, void*);
 extern "C" int eqd_attention_tc(const eqd_graph*, const float*, const void*, float*, void*);
 
-extern "C" int eqd_node_stage_tc(const eqd_graph* g, const eqd_layer* p_l, const eqd_layer* p_next_l,
-                                 const float* h_in, const float* h0, const float* proj, const float* aggr, void* kv,
-                                 float* mu, float* h_out, float* proj_next, void* stream) {
+namespace eqd {
+int node_stage_tc(const eqd_graph* g, const eqd_layer* p_l, const eqd_layer* p_next_l, const float* h_in, const float* h0,
+                  const float* proj, const float* aggr, void* kv, float* mu, float* h_out, float* proj_next,
+                  const DropoutArgs* drop, void* stream) {
   const eqd_layer_params* p = p_l ? &p_l->dev : nullptr;
   const eqd_layer_params* p_next = p_next_l ? &p_next_l->dev : nullptr;
   if (!g || !p || !kv || !mu) return EQD_ERR_BAD_ARG;
   if (p_next && !proj_next) return EQD_ERR_BAD_ARG;
   int rc = eqd_attention_tc(g, proj, kv, mu, stream);
   if (rc) return rc;
-  rc = eqd_node_mlp_tc(g, p_l, h_in, aggr, mu, h0, h_out, stream);
+  rc = node_mlp_tc(g, p_l, h_in, aggr, mu, h0, h_out, drop, stream);
   if (rc) return rc;
   if (p_next) rc = eqd_project_tc(g, p_next_l, h_out, proj_next, kv, stream);
   return rc;
+}
+}  // namespace eqd
+
+extern "C" int eqd_node_stage_tc(const eqd_graph* g, const eqd_layer* p_l, const eqd_layer* p_next_l,
+                                 const float* h_in, const float* h0, const float* proj, const float* aggr, void* kv,
+                                 float* mu, float* h_out, float* proj_next, void* stream) {
+  return eqd::node_stage_tc(g, p_l, p_next_l, h_in, h0, proj, aggr, kv, mu, h_out, proj_next, nullptr, stream);
 }

@@ -435,19 +435,27 @@ class IEGMNEngine:
 
     def forward(self, plan: GraphPlan, emb: torch.Tensor, layers: List[PackedLayer], head: PackedHead,
                 res_l, res_r, mu_l, mu_r, x_l, x_r, check_status: bool = True, log=None,
-                stage_timer=None, record_event: bool = True, train_stash=None) -> Dict[str, torch.Tensor]:
+                stage_timer=None, record_event: bool = True, train_stash=None, dropout_p: float = 0.0,
+                dropout_rank: int = 0) -> Dict[str, torch.Tensor]:
         """One forward = ONE call into the library (eqd_iegmn_forward): the per-stage entry points are chained in C on
         the current stream out of a single workspace allocation.  EQD_PY_FORWARD=1 selects the stage-by-stage Python
-        driver below instead (same kernels; used to A/B the two and by the per-stage tests)."""
+        driver below instead (same kernels; used to A/B the two and by the per-stage tests).
+
+        ``dropout_p`` > 0 (training): a fresh 64-bit key is drawn on the device for this call (``nat.Dropout``) and the
+        forward applies the four dropout sites (eqd_iegmn_forward_dropout); the key travels in ``out['dropout']`` so that the
+        backward regenerates the same masks.  ``dropout_rank`` separates the masks of data-parallel ranks."""
         with torch.cuda.device(self.device):   # the raw launches below go to the CURRENT device: make it the model's
+            drop = nat.Dropout(dropout_p, self.device, dropout_rank) if dropout_p > 0 else None
             if _PY_FORWARD:
+                if drop is not None:
+                    raise NotImplementedError('dropout runs through eqd_iegmn_forward_dropout only (unset EQD_PY_FORWARD)')
                 return self._forward_py(plan, emb, layers, head, res_l, res_r, mu_l, mu_r, x_l, x_r, check_status, log,
                                         stage_timer)
             return self._forward_native(plan, emb, layers, head, res_l, res_r, mu_l, mu_r, x_l, x_r, check_status, log,
-                                        stage_timer, record_event, train_stash)
+                                        stage_timer, record_event, train_stash, drop)
 
     def _forward_native(self, plan, emb, layers, head, res_l, res_r, mu_l, mu_r, x_l, x_r, check_status, log,
-                        stage_timer, record_event=True, train_stash=None):
+                        stage_timer, record_event=True, train_stash=None, drop=None):
         lib, dev = self.lib, self.device
         st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         N, B = plan.N, plan.n_pairs
@@ -478,8 +486,13 @@ class IEGMNEngine:
         events = stage_timer.new_forward(len(layers)) if stage_timer is not None else None
         io.stage_events = C.cast(events, C.c_void_p) if events is not None else None
         larr = (C.POINTER(nat.EqdLayer) * len(layers))(*[C.pointer(l.struct) for l in layers])
-        nat.check(lib.eqd_iegmn_forward(g, larr, len(layers), C.byref(head.struct), C.byref(io), nat.ptr(ws),
-                                        plan.forward_ws_bytes, st), 'eqd_iegmn_forward')
+        if drop is None:
+            nat.check(lib.eqd_iegmn_forward(g, larr, len(layers), C.byref(head.struct), C.byref(io), nat.ptr(ws),
+                                            plan.forward_ws_bytes, st), 'eqd_iegmn_forward')
+        else:
+            nat.check(lib.eqd_iegmn_forward_dropout(g, larr, len(layers), C.byref(head.struct), C.byref(io),
+                                                    C.byref(drop.struct), nat.ptr(ws), plan.forward_ws_bytes, st),
+                      'eqd_iegmn_forward_dropout')
         kab = lambda mask: nat.check(lib.eqd_kabsch_apply(
             g, nat.ptr(cov), nat.ptr(ymean), nat.ptr(x_l), nat.ptr(mask), nat.ptr(rot), nat.ptr(trans),
             nat.ptr(lig_out), nat.ptr(sing), nat.ptr(status), st), 'eqd_kabsch_apply')
@@ -493,7 +506,8 @@ class IEGMNEngine:
             status_event.record()
         out = {'status_lease': lease, 'ligand_coors': lig_out, 'keypts': keyp, 'rotation': rot, 'translation': trans,
                'h': h_fin, 'x64': x_fin, 'cov': cov, 'sing': sing, 'status': status, 'unsorted': plan.unsorted,
-               'kabsch': kab, 'status_host': status_host, 'status_event': status_event, '_keep': (ws, ymean, x_l)}
+               'kabsch': kab, 'status_host': status_host, 'status_event': status_event, '_keep': (ws, ymean, x_l),
+               'dropout': drop}
         if check_status:
             self.resolve_status(plan, out, kab, log)
         return out

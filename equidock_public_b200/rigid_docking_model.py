@@ -17,10 +17,18 @@ checkpoints load with ``strict=True``.  The graph argument may be a batched DGL 
 
 Scope of this engine: forward AND backward of the configuration the shipped checkpoints use
 (``nonlin='lkyrelu'``, ``layer_norm='LN'``, ``layer_norm_coors='0'``, ``final_h_layer_norm='0'``,
-``cross_msgs``, ``use_dist_in_layers``, ``rot_model='kb_att'``, ``fine_tune=False``, dropout inactive).
+``cross_msgs``, ``use_dist_in_layers``, ``rot_model='kb_att'``, ``fine_tune=False``), with any ``dropout`` in [0, 1).
 Anything else raises ``NotImplementedError``; a missing CUDA library raises -- there is no CPU path.
 In training mode (``model.train()`` with grad enabled) the outputs of ``Rigid_Body_Docking_Net.forward`` are
 autograd-connected: the whole path is one autograd node backed by the CUDA backward kernels (``training.py``).
+
+Dropout: in ``train()`` mode with 0 < p < 1, ``Rigid_Body_Docking_Net.forward`` and ``IEGMN.forward`` apply the four
+``nn.Dropout`` sites (edge_mlp, coors_mlp, node_mlp, mlp_h_mean_ROT), with or without grad enabled; p is read from the
+``nn.Dropout`` modules at call time (they must agree).  Masks are counter-based (Philox4x32-10, ``include/eqd_iegmn.h``
+``eqd_dropout``) under a 64-bit key drawn per call from torch's CUDA generator, so ``torch.manual_seed`` reproduces a run
+and the CPU generator is left alone; they are statistically, not bitwise, torch's.  The per-layer operator
+``IEGMN_Layer.forward`` and the inference tools (``graphed()``, ``serving``, ``graph_build``) keep raising
+``NotImplementedError`` in that mode.
 """
 import math  # noqa: F401  (re-exported, see module docstring)
 import sys  # noqa: F401
@@ -313,14 +321,34 @@ class IEGMN(nn.Module):
             self._head_key = key
         return self._head
 
-    def run_engine(self, batch_hetero_graph, check_status=True, record_event=True):
+    def dropout_p(self) -> float:
+        """The dropout probability the next forward applies: p of the model's ``nn.Dropout`` modules that are in training
+        mode (0 when none is).  Raises NotImplementedError when active modules disagree or p >= 1."""
+        mods = [m for lay in self.iegmn_layers for m in (lay.edge_mlp[1], lay.coors_mlp[1], lay.node_mlp[1])]
+        mods.append(self.mlp_h_mean_ROT[1])
+        ps = {float(m.p) if m.training else 0.0 for m in mods}
+        if len(ps) > 1:
+            raise NotImplementedError(f'dropout probabilities / modes differ between the nn.Dropout modules ({sorted(ps)}): '
+                                      'the CUDA engine applies one p to all four sites')
+        p = ps.pop()
+        if p >= 1.0:
+            raise NotImplementedError(f'dropout p={p} >= 1 is not implemented in the CUDA engine')
+        return p
+
+    def run_engine(self, batch_hetero_graph, check_status=True, record_event=True, allow_dropout=False):
         """The whole hot path on the device; returns the engine's raw output dict.  With ``check_status=False`` the
         per-pair status words are left pending (``resolve(out)`` finishes the call).  ``record_event=False`` is for
-        CUDA-graph capture (``graphed.GraphedForward``), which records its own completion event per replay."""
+        CUDA-graph capture (``graphed.GraphedForward``), which records its own completion event per replay.
+        ``allow_dropout`` (``IEGMN.forward``): apply dropout in train() mode; otherwise that mode raises, as in the
+        inference tools built on this call."""
         emb = self.residue_emb_layer.weight
         dev = emb.device
-        for lay in self.iegmn_layers:
-            lay._check_mode()
+        drop_p = 0.0
+        if allow_dropout:
+            drop_p = self.dropout_p()
+        else:
+            for lay in self.iegmn_layers:
+                lay._check_mode()
         eng = IEGMNEngine(dev)
         layers = [lay.packed(dev) for lay in self.iegmn_layers]
         head = self.packed_head(dev)
@@ -329,13 +357,14 @@ class IEGMN(nn.Module):
         emb32 = emb.detach().to(torch.float32).contiguous()
         call = lambda p, chk: eng.forward(p, emb32, layers, head, nl['res_feat'], nr['res_feat'], nl['mu_r_norm'],
                                           nr['mu_r_norm'], nl['new_x'], nr['x'], chk, self.log,
-                                          record_event=record_event)
+                                          record_event=record_event, dropout_p=drop_p)
         try:
             out = call(plan, check_status)
         except UnsortedEdges:
             plan = _sorted_plan(batch_hetero_graph, dev, self.graph_max_neighbor)
             out = call(plan, True)
         out['plan'], out['engine'], out['graph'] = plan, eng, batch_hetero_graph
+        out['allow_dropout'] = allow_dropout
         return out
 
     def resolve(self, out):
@@ -345,12 +374,12 @@ class IEGMN(nn.Module):
             out['engine'].resolve_status(out['plan'], out, out['kabsch'], self.log)
             return out
         except UnsortedEdges:
-            return self.run_engine(out['graph'], True)
+            return self.run_engine(out['graph'], True, allow_dropout=out.get('allow_dropout', False))
 
     def forward(self, batch_hetero_graph, epoch):
         """Returns ``[T list, b list, Y_ligand list, Y_receptor list]`` like the reference (:602) and
-        writes ``x_iegmn_out`` / ``hv_iegmn_out`` into the graph (:507-510)."""
-        return self.package(self.run_engine(batch_hetero_graph), batch_hetero_graph)
+        writes ``x_iegmn_out`` / ``hv_iegmn_out`` into the graph (:507-510).  Applies dropout in train() mode."""
+        return self.package(self.run_engine(batch_hetero_graph, allow_dropout=True), batch_hetero_graph)
 
     def package(self, out, batch_hetero_graph):
         plan = out['plan']

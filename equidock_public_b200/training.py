@@ -193,6 +193,7 @@ class TrainEngine:
         self._maps: Dict[int, dict] = {}
         self._ws: Optional[BackwardWorkspace] = None
         self._head_maps = None
+        self.rank = 0   # data-parallel rank: the fourth word of the dropout counter (DataParallelTrainer sets it)
 
     # ---- packs ----------------------------------------------------------------------------------------------------
     def layer_pack(self, lay_module) -> LayerTrainPack:
@@ -221,15 +222,14 @@ class TrainEngine:
     def forward(self, graph, log=None):
         from .rigid_docking_model import _plan_for, _sorted_plan, UnsortedEdges
         iegmn, dev, lib = self.iegmn, self.device, self.lib
-        for lay in iegmn.iegmn_layers:
-            lay._check_mode()
+        p = iegmn.dropout_p()   # > 0 in train() mode with dropout: masks drawn per call, regenerated by backward()
         plan = _plan_for(graph, dev, iegmn.graph_max_neighbor)
         try:
-            return self._forward_plan(graph, plan, log)
+            return self._forward_plan(graph, plan, log, p)
         except UnsortedEdges:
-            return self._forward_plan(graph, _sorted_plan(graph, dev, iegmn.graph_max_neighbor), log)
+            return self._forward_plan(graph, _sorted_plan(graph, dev, iegmn.graph_max_neighbor), log, p)
 
-    def _forward_plan(self, graph, plan, log):
+    def _forward_plan(self, graph, plan, log, dropout_p=0.0):
         from .hetero_graph import LIGAND, RECEPTOR
         iegmn, dev, lib = self.iegmn, self.device, self.lib
         layers = [lay.packed(dev) for lay in iegmn.iegmn_layers]
@@ -245,7 +245,8 @@ class TrainEngine:
             eng = IEGMNEngine(dev)
             emb32 = iegmn.residue_emb_layer.weight.detach().to(_f32).contiguous()
             out = eng.forward(plan, emb32, layers, head, nl['res_feat'], nr['res_feat'], nl['mu_r_norm'], nr['mu_r_norm'],
-                              nl['new_x'], nr['x'], True, log, train_stash=stash)
+                              nl['new_x'], nr['x'], True, log, train_stash=stash, dropout_p=dropout_p,
+                              dropout_rank=self.rank)
         out.update(plan=plan, engine=eng, graph=graph, stash=stash, stash_offsets=list(offs), layers=layers, head=head,
                    res_l=nl['res_feat'].to(_f32).contiguous(), res_r=nr['res_feat'].to(_f32).contiguous(),
                    x_lig_in=nl['new_x'].to(_f32).contiguous())
@@ -291,11 +292,13 @@ class TrainEngine:
             gq = flat[off['iegmn_original.att_mlp_query_ROT.0.weight']:]
             dh_cur, dh_nxt = ws.dh
             dx_cur, dx_nxt = ws.dx
-            nat.check(lib.eqd_bwd_head(g, C.byref(fwd['head'].struct), nat.ptr(fwd['h']), nat.ptr(fwd['x64']),
-                                       nat.ptr(fwd['cov']), nat.ptr(fwd['x_lig_in']), nat.ptr(d_coors), nat.ptr(d_keypts),
-                                       nat.ptr(d_rot), nat.ptr(d_trans), nat.ptr(ws.head_ws), ws.head_ws_bytes,
-                                       nat.ptr(dh_cur), nat.ptr(dx_cur), nat.ptr(ws.dpre), nat.ptr(gk), nat.ptr(gq), st),
-                      'eqd_bwd_head')
+            drop = fwd.get('dropout')   # the forward's masks, regenerated from its key (NULL: no dropout)
+            dref = C.byref(drop.struct) if drop is not None else None
+            nat.check(lib.eqd_bwd_head_dropout(g, C.byref(fwd['head'].struct), nat.ptr(fwd['h']), nat.ptr(fwd['x64']),
+                                               nat.ptr(fwd['cov']), nat.ptr(fwd['x_lig_in']), nat.ptr(d_coors),
+                                               nat.ptr(d_keypts), nat.ptr(d_rot), nat.ptr(d_trans), nat.ptr(ws.head_ws),
+                                               ws.head_ws_bytes, nat.ptr(dh_cur), nat.ptr(dx_cur), nat.ptr(ws.dpre),
+                                               nat.ptr(gk), nat.ptr(gq), dref, L, st), 'eqd_bwd_head')
             if capture is not None:
                 capture.append({'head': True, 'dh': dh_cur.reshape(-1)[:N * 64].clone().view(N, 64), 'dx': dx_cur.clone()})
             hm = self.head_maps()
@@ -327,10 +330,11 @@ class TrainEngine:
                 ldmu = nat.H0_PAD if dh == nat.H0 else nat.HID
                 nat.check(lib.eqd_project(g, lp, h_in, ldh, nat.ptr(ws.proj), st), 'eqd_project')
                 nparts = C.c_int32(0)
-                nat.check(lib.eqd_bwd_node_mlp(g, lp, nat.ptr(tp.t['w_node1_lin']), nat.ptr(tp.t['w_node2_lin']), h_in, ldh,
-                                               aggr, mu, ldmu, h0_ptr, nat.ptr(dh_cur), nat.ptr(dh_nxt), nat.ptr(ws.daggr),
-                                               nat.ptr(ws.dmu), nat.ptr(ws.dh0), nat.ptr(ws.n5), nat.ptr(ws.du),
-                                               nat.ptr(ws.vec), C.byref(nparts), st), 'eqd_bwd_node_mlp')
+                nat.check(lib.eqd_bwd_node_mlp_dropout(g, lp, nat.ptr(tp.t['w_node1_lin']), nat.ptr(tp.t['w_node2_lin']),
+                                                       h_in, ldh, aggr, mu, ldmu, h0_ptr, nat.ptr(dh_cur), nat.ptr(dh_nxt),
+                                                       nat.ptr(ws.daggr), nat.ptr(ws.dmu), nat.ptr(ws.dh0), nat.ptr(ws.n5),
+                                                       nat.ptr(ws.du), nat.ptr(ws.vec), C.byref(nparts), dref, li, st),
+                          'eqd_bwd_node_mlp')
                 self._reduce(ws.vec, nparts.value, 144, tp.maps['nodevec'], flat, st)
                 # node MLP weight gradients
                 sk = float(lp_obj.struct.dev.skip_weight_h) if dh == nat.HID else 1.0
@@ -347,10 +351,11 @@ class TrainEngine:
                         self._reduce(ws.colsum, nchx.value, dhp, tp.maps['node1_bias'], flat, st)
                 nat.check(lib.eqd_bwd_attention(g, lp, nat.ptr(ws.proj), mu, ldmu, nat.ptr(ws.dmu), nat.ptr(ws.dP),
                                                 nat.ptr(ws.rowstat), st), 'eqd_bwd_attention')
-                nat.check(lib.eqd_bwd_edge(g, lp, nat.ptr(tp.t['w2lin']), nat.ptr(tp.t['w3lin']), nat.ptr(ws.proj), x_in,
-                                           nat.ptr(ws.daggr), nat.ptr(dx_cur), nat.ptr(ws.ein), nat.ptr(ws.n1),
-                                           nat.ptr(ws.msg), nat.ptr(ws.dz3), nat.ptr(ws.dmsg), nat.ptr(ws.dz1),
-                                           nat.ptr(ws.dxrel), nat.ptr(ws.vec), C.byref(nparts), st), 'eqd_bwd_edge')
+                nat.check(lib.eqd_bwd_edge_dropout(g, lp, nat.ptr(tp.t['w2lin']), nat.ptr(tp.t['w3lin']), nat.ptr(ws.proj),
+                                                   x_in, nat.ptr(ws.daggr), nat.ptr(dx_cur), nat.ptr(ws.ein), nat.ptr(ws.n1),
+                                                   nat.ptr(ws.msg), nat.ptr(ws.dz3), nat.ptr(ws.dmsg), nat.ptr(ws.dz1),
+                                                   nat.ptr(ws.dxrel), nat.ptr(ws.vec), C.byref(nparts), dref, li, st),
+                          'eqd_bwd_edge')
                 self._reduce(ws.vec, nparts.value, 256, tp.maps['edgevec'], flat, st)
                 nch = self._tn(ws, ws.ein, 44, 44, ws.dz1, 64, 64, E, 1.0, False, st)
                 self._reduce(ws.partial, nch, 44 * 64, tp.maps['edge1'], flat, st)
@@ -467,6 +472,11 @@ class DataParallelTrainer:
         self.loss_args = (pocket_ot_loss_weight, intersection_loss_weight, intersection_sigma, intersection_surface_ct)
         self.steps = 0
         self.comm = torch.cuda.Stream(dev) if self.world > 1 else None
+        self.rank = 0
+        if self.world > 1:
+            import torch.distributed as dist
+            self.rank = dist.get_rank(group)
+        self.engine.rank = self.rank   # equally seeded ranks draw different dropout masks
         self.lib = nat.load()
 
     def invalidate_packed(self):

@@ -32,7 +32,7 @@
 extern "C" {
 #endif
 
-#define EQD_ABI_VERSION 8
+#define EQD_ABI_VERSION 9
 
 #define EQD_EDGE_FEATS 27     /* input_edge_feats_dim, protein_utils.py:71-86 + :373-389 */
 #define EQD_N_RBF 15          /* all_sigmas_dist = 1.5**s, rigid_docking_model.py:116 */
@@ -324,6 +324,30 @@ int eqd_iegmn_forward(const eqd_graph* g, const eqd_layer* const* layers, int32_
                       const eqd_head_params* hp, const eqd_forward_io* io, void* workspace, size_t workspace_bytes,
                       void* stream);
 
+/* ---- dropout in training (the four nn.Dropout sites of rigid_docking_model.py :119-159, 427-438) --------------------------
+ * Counter-based masks, so that the backward regenerates the forward's mask and nothing is stored.  Element (row, col) of
+ * site s in layer l is kept iff word (col % 4) of Philox4x32-10(counter = {col / 4, row, 4 l + s, rank}, key = {*key low 32
+ * bits, high 32 bits}) >= threshold; a kept element is multiplied by `scale`, a dropped one by 0.  Sites: 0 edge_mlp (after
+ * its first Linear, 64 wide), 1 coors_mlp (64), 2 node_mlp (64; 69 in the 69-wide layer 0), 3 mlp_h_mean_ROT (64, layer =
+ * n_layers).  Rows: global edge id in CSR order (sites 0, 1), global node id (sites 2, 3).  The mask multiplies the LeakyReLU
+ * output, which equals the reference's dropout-then-LeakyReLU (LeakyReLU is positively homogeneous).
+ * A NULL descriptor means no dropout: the entry points below then run exactly the kernels of the inference path.          */
+typedef struct eqd_dropout {
+  const uint64_t* key;        /* DEVICE memory: the 64-bit key of this forward (read by the kernels, no host sync) */
+  uint32_t threshold;         /* min(round(p 2^32), 2^32 - 1) */
+  float scale;                /* fp32(1 / (1 - p)) */
+  uint32_t rank;              /* data-parallel rank: equally seeded ranks draw different masks */
+} eqd_dropout;
+
+/* eqd_iegmn_forward with dropout (tensor-core path only: EQD_ERR_UNSUPPORTED with io->layer0_fp32 or a layer without
+ * tensor-core panels, whose fp32 CUDA-core twins have no dropout). */
+int eqd_iegmn_forward_dropout(const eqd_graph* g, const eqd_layer* const* layers, int32_t n_layers,
+                              const eqd_head_params* hp, const eqd_forward_io* io, const eqd_dropout* dropout,
+                              void* workspace, size_t workspace_bytes, void* stream);
+/* keep[r][c] = 1 / 0 for rows 0..rows-1, columns 0..cols-1 of (layer, site) (device memory; for tests and oracles). */
+int eqd_dropout_mask(const eqd_dropout* dropout, int32_t layer, int32_t site, int32_t rows, int32_t cols, uint8_t* keep,
+                     void* stream);
+
 /* =====================================================================================================================
  * BACKWARD of the path (training: BASELINE configs 3-4).  The reference has no backward code: these entry points are
  * what a binding would call from torch.autograd.Function.backward in place of `loss.backward()` (src/train.py:154)
@@ -355,6 +379,12 @@ int eqd_bwd_node_mlp(const eqd_graph* g, const eqd_layer* p, const float* w_node
                      const float* h_in, int32_t ldh, const float* aggr, const float* mu, int32_t ldmu, const float* h0,
                      const float* dh_out, float* dh_in, float* daggr, float* dmu, float* dh0_acc, float* n5_out,
                      float* du_out, float* vec_partial /* [148][144] */, int32_t* n_partials_out, void* stream);
+/* Same, regenerating the forward's site-2 mask of layer `layer` (dropout NULL = eqd_bwd_node_mlp). */
+int eqd_bwd_node_mlp_dropout(const eqd_graph* g, const eqd_layer* p, const float* w_node1_lin, const float* w_node2_lin,
+                             const float* h_in, int32_t ldh, const float* aggr, const float* mu, int32_t ldmu,
+                             const float* h0, const float* dh_out, float* dh_in, float* daggr, float* dmu, float* dh0_acc,
+                             float* n5_out, float* du_out, float* vec_partial, int32_t* n_partials_out,
+                             const eqd_dropout* dropout, int32_t layer, void* stream);
 /* Cross attention backward (:46-64, 247-256): dmu [n][dhp] -> dP[:, 128:] = [dQpre | dKpre | dV] of the combined
  * projection-gradient matrix dP [n][128 + 3 dhp].  proj = this layer's fp32 projections (eqd_project), mu the stashed
  * attention output, rowstat [n][4] scratch.                                                                         */
@@ -368,6 +398,12 @@ int eqd_bwd_edge(const eqd_graph* g, const eqd_layer* p, const float* w2lin, con
                  const double* x_in, const float* daggr, const double* dx_out, float* ein_out, float* n1_out,
                  float* msg_out, float* dz3_out, float* dmsg_out, float* dz1_out, double* dxrel_out,
                  float* vec_partial /* [148][256] */, int32_t* n_partials_out, void* stream);
+/* Same, regenerating the forward's site-0 / site-1 masks of layer `layer` (dropout NULL = eqd_bwd_edge). */
+int eqd_bwd_edge_dropout(const eqd_graph* g, const eqd_layer* p, const float* w2lin, const float* w3lin, const float* proj,
+                         const double* x_in, const float* daggr, const double* dx_out, float* ein_out, float* n1_out,
+                         float* msg_out, float* dz3_out, float* dmsg_out, float* dz1_out, double* dxrel_out,
+                         float* vec_partial, int32_t* n_partials_out, const eqd_dropout* dropout, int32_t layer,
+                         void* stream);
 /* Per node: dP[:, 0:64] = sum over OUT-edges of dz1, dP[:, 64:128] = sum over IN-edges, dx_in = (1 - eta) dx_out +
  * sum_out dxrel - sum_in dxrel.  out_ptr [n+1] / out_edge [E]: edges grouped by SOURCE node (ascending edge id).      */
 int eqd_bwd_edge_gather(const eqd_graph* g, const int32_t* out_ptr, const int32_t* out_edge, const float* dz1,
@@ -386,6 +422,11 @@ int eqd_bwd_head(const eqd_graph* g, const eqd_head_params* hp, const float* h, 
                  const float* x_lig_in, const float* dcoors, const double* dkeypts, const float* drot,
                  const float* dtrans, void* workspace, size_t workspace_bytes, float* dh, double* dx, float* dpre,
                  float* g_wkey, float* g_wquery, void* stream);
+/* Same, regenerating the forward's site-3 mask; `layer` = the model's number of IEGMN layers (dropout NULL = eqd_bwd_head). */
+int eqd_bwd_head_dropout(const eqd_graph* g, const eqd_head_params* hp, const float* h, const double* x, const double* cov,
+                         const float* x_lig_in, const float* dcoors, const double* dkeypts, const float* drot,
+                         const float* dtrans, void* workspace, size_t workspace_bytes, float* dh, double* dx, float* dpre,
+                         float* g_wkey, float* g_wquery, const eqd_dropout* dropout, int32_t layer, void* stream);
 
 /* ---- training losses on the device (src/train.py:41-49, 112-150; src/utils/ot_utils.py:5-29) ------------------------
  * Per pair: MSE of the predicted ligand coordinates, body-intersection loss, pocket OT loss with the EXACT earth mover's
